@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the batched MiniWorld step path on B200 (and the CPU arm).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json): MiniWorld-FourRooms-v0, N_envs = 4096 per GPU, 80x60 RGB + depth,
 uniformly random actions, next-step auto-reset, env i seeded 1000 + i.  One "step" = one
@@ -17,6 +17,11 @@ mwb_step call: K1 (physics / reward / device resets) + K2 (render RGB + depth) f
   roofline: K2's algorithmic bytes (framebuffer written once) / its CUDA-event time inside the
            timed region, against the measured HBM copy bandwidth (MEASURED_PEAKS.json).
   cpu_baseline: the oracle port (oracle/physics_port.py + oracle/softgl.c) on host cores.
+
+--dump-outputs DIR: after the timed steps, what the last timed step returned (obs, reward, terminated, truncated and
+the info arrays, e.g. depth) is written as DIR/<name>.npy in float32 (float64 where the step returns float64), for
+a fixed, seeded sample of envs that keeps the files under 64 MB (DIR/env_index.npy lists it).  Actions and seeds
+depend only on the arguments, so two builds run with the same arguments can be compared output for output.
 
 --impl reference: the reference's own Pyglet/OpenGL path cannot run here (no pyglet, GL or
 gymnasium in the image; /root/reference is absent on the GPU box), so this arm times the CPU
@@ -41,6 +46,7 @@ W, H = 80, 60
 BYTES_RGB = W * H * 3
 BYTES_DEPTH = W * H * 4
 FALLBACK_HBM_GBS = 6650.0
+DUMP_BYTES = 60 << 20               # --dump-outputs payload limit (64 MB with headroom for the .npy headers)
 # BASELINE.json configs (index as in its `configs` list); envs = per GPU under weak scaling.  Config 3 is the one the
 # metric is quoted on and the default; 4 and 5 are the two configs it states for 8 GPUs (8192 / 8 and 4096 / 8 envs per GPU).
 CONFIGS = {
@@ -265,6 +271,25 @@ def run_reference_arm(args):
 
 # --------------------------------------------------------------------------- GPU arm
 
+def dump_outputs(path, step_out):
+    """Write the arrays one BatchedMiniWorld.step returned (see --dump-outputs) to path/<name>.npy."""
+    import torch
+    obs, reward, terminated, truncated, info = step_out
+    arrays = dict(obs=obs, reward=reward, terminated=terminated, truncated=truncated, **info)
+    n = obs.shape[0]
+    for k, v in arrays.items():
+        assert v.shape[0] == n, "%s is not per env" % k
+    wide = lambda v: torch.float64 if v.dtype == torch.float64 else torch.float32
+    env_bytes = sum(v[0].numel() * (8 if wide(v) == torch.float64 else 4) for v in arrays.values())
+    keep = min(n, DUMP_BYTES // env_bytes)
+    rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False)) if keep < n else np.arange(n)
+    idx = torch.as_tensor(rows, device=obs.device)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "env_index.npy"), rows.astype(np.float64))
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v.index_select(0, idx).to(wide(v)).cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -316,10 +341,10 @@ def run_ours(args):
     def one_step(t):
         if peer:                          # K2 writes into rank 0's HBM over NVLink; one-way completion flags, no collective
             return sharded.step_peer(acts[t])
-        obs, rew, te, tr, info = env.step(acts[t])
+        out = env.step(acts[t])
         if world > 1:
-            dist.gather(obs, gather_list, dst=0)
-        return obs
+            dist.gather(out[0], gather_list, dst=0)
+        return out
 
     # ---- device-resident arm
     for t in range(Wm):
@@ -334,7 +359,7 @@ def run_ours(args):
     done0 = int(env.get_state()["episodes_done"][0])
     e0.record()
     for t in range(Wm, total):
-        one_step(t)
+        last = one_step(t)
     e1.record()
     barrier()
     sampler.stop_flag = True
@@ -343,6 +368,8 @@ def run_ours(args):
     env.engine.profile(False)
     done_steps = int(env.get_state()["episodes_done"][0]) - done0
     launches = env.engine.launch_count() - launches0
+    if args.dump_outputs:                  # before the end-to-end arm below steps the same buffers again
+        dump_outputs(args.dump_outputs, last)
     if world > 1:
         tmax = torch.tensor([ms], dtype=torch.float64, device=dev)
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
@@ -465,7 +492,12 @@ def main():
     ap.add_argument("--no-numa", action="store_true", help="do not bind the process to the GPU's NUMA node")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--nccl-gather", action="store_true", help="gather observations with NCCL instead of peer stores")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl ours in a single process")
     if args.warmup < 3:
         args.warmup = 3
     claim_stdout()

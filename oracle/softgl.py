@@ -280,6 +280,15 @@ def render(env, texset, tex_index, width=80, height=60, samples=8, want_codes=Fa
     return _run(env, texset, draw_list(env, tex_index), width, height, samples, want_codes=want_codes)
 
 
+def light_position(env):
+    """The four GLfloats of GL_LIGHT0's position as the reference passes them."""
+    # glLightfv(GL_LIGHT0, GL_POSITION, (GLfloat * 4)(*self.light_pos + [1])) (miniworld.py:1031), restated
+    # literally: light_pos is an ndarray (params.py:45-46), so `+ [1]` adds 1 to each component, three GLfloats are
+    # passed and w stays 0 -- a DIRECTIONAL light along light_pos + 1.  (A plain list would give a positional light.)
+    lp = list(env.light_pos + [1])
+    return [float(f32(v)) for v in lp] + [0.0] * (4 - len(lp))
+
+
 def _run(env, texset, lst, width, height, samples, want_codes=False, ortho=None, query=None, query_out=None):
     pos, nrm, uv, rgb, tx = lst
     sc = _Scene()
@@ -295,11 +304,7 @@ def _run(env, texset, lst, width, height, samples, want_codes=False, ortho=None,
         sc.sky[k] = float(env.sky_color[k])
         sc.light_color[k] = float(env.light_color[k])
         sc.light_ambient[k] = float(env.light_ambient[k])
-    # glLightfv(GL_LIGHT0, GL_POSITION, (GLfloat * 4)(*self.light_pos + [1])) (miniworld.py:1031), restated
-    # literally: light_pos is an ndarray (params.py:45-46), so `+ [1]` adds 1 to each component, three GLfloats are
-    # passed and w stays 0 -- a DIRECTIONAL light along light_pos + 1.  (A plain list would give a positional light.)
-    lp = list(env.light_pos + [1])
-    lp = [float(f32(v)) for v in lp] + [0.0] * (4 - len(lp))
+    lp = light_position(env)
     for k in range(3):
         sc.light_pos[k] = lp[k]
     sc.light_w = lp[3]

@@ -1,21 +1,30 @@
 """Pixel parity pinned to the reference's own GL stream.
 
-(1) Where /root/reference exists: the UNMODIFIED reference runs under the recording fixed-function GL
-    (oracle/gl_record.py); the frames its render_obs() / render_depth() / render_top_view() / get_visible_ents()
-    return -- the rasterised stream of the GL calls it made -- must equal, bit for bit, oracle/softgl.py's rendering
-    of the package's mirror objects in the same state.  All 23 reference ids (+ the MazeS8 alias), with and without
-    domain randomisation.
-(2) Everywhere (no reference needed): the kernels' arithmetic compiled for the CPU (tests/hostsim) replays the
-    golden trajectories and is compared with the committed frames the reference returned (tests/golden/stream_*.npz).
+(1) The UNMODIFIED reference, run under the recording fixed-function GL (oracle/gl_record.py), returned frames from
+    its render_obs() / render_depth() / render_top_view() / render() and sets from get_visible_ents() -- the
+    rasterised stream of the GL calls it made.  oracle/gen_mirror_golden.py stored, for each of those frames, the
+    reference's dynamic state and a digest of what it returned (tests/golden/mirror_frames.npz); here the package's
+    mirror objects are put into each stored state and oracle/softgl.py's rendering of them must equal the reference's
+    frame bit for bit.  All 23 reference ids (+ the MazeS8 alias), with and without domain randomisation.
+(2) The kernels' arithmetic compiled for the CPU (tests/hostsim) replays the golden trajectories and is compared with
+    the committed frames the reference returned (tests/golden/stream_*.npz).
 The same comparison through libmwb.so on a B200 is tests/test_gpu_stream.py.
 """
+import os
+
 import numpy as np
 import pytest
 
+from conftest import GOLDEN
 from helpers import stream_cases, stream_parity
-from oracle import ref_stub
+from oracle import softgl
+from oracle.stream_check import Mirror, frame_digest, load_frames, replay
 
-needs_reference = pytest.mark.skipif(not ref_stub.reference_available(), reason="needs /root/reference")
+
+@pytest.fixture(scope="module")
+def recorded():
+    with np.load(os.path.join(GOLDEN, "mirror_frames.npz")) as z:
+        return {k: z[k] for k in z.files}
 
 
 def _levels():
@@ -23,84 +32,78 @@ def _levels():
     return level_ids()
 
 
-@needs_reference
 @pytest.mark.parametrize("level", _levels())
-def test_reference_gl_stream_equals_mirror(softgl_lib, level):
-    from oracle.stream_check import compare
+def test_reference_gl_stream_equals_mirror(softgl_lib, recorded, level):
     for dr in (False, True):
         if dr and level == "MiniWorld-Sign-v0":
             continue                                  # Sign fixes domain_rand=False itself (sign.py:88-93)
-        n, bad, worst, dbad = compare(level, dr, steps=12)
-        assert n == 13 and bad == 0 and dbad == 0, "%s dr=%d: %d / %d frames differ (worst %d LSB), %d depth maps differ" % (
-            level, dr, bad, n, worst, dbad)
+        m = Mirror(level, dr)
+        n = bad = dbad = 0
+        for f in replay(m, load_frames(recorded, "stream %s %d" % (level, dr))):
+            rgb, depth = m.mirror_frame()
+            n += 1
+            bad += not np.array_equal(frame_digest(rgb), f["digest"][0])
+            dbad += not np.array_equal(frame_digest(depth), f["digest"][1])
+        assert n == 13 and bad == 0 and dbad == 0, "%s dr=%d: %d / %d frames differ, %d depth maps differ" % (
+            level, dr, bad, n, dbad)
 
 
-@needs_reference
 @pytest.mark.parametrize("level", ["MiniWorld-Hallway-v0", "MiniWorld-PickupObjects-v0", "MiniWorld-ThreeRooms-v0",
                                    "MiniWorld-Sidewalk-v0", "MiniWorld-Sign-v0"])
-def test_reference_other_views_equal_mirror(softgl_lib, level):
+def test_reference_other_views_equal_mirror(softgl_lib, recorded, level):
     """render_top_view (with the agent marker and its leaked normal), get_visible_ents, a 160 x 120 observation."""
-    from oracle.stream_check import Pair
-    p = Pair(level, False, obs_width=160, obs_height=120)
-    rng = np.random.default_rng(7)
-    p.reset(11)
-    for t in range(6):
-        obs, _, term, trunc, _ = p.step(int(rng.integers(0, p.ref.action_space.n)))
-        if term or trunc:
-            p.reset(12 + t)
-            continue
-        obs = obs["obs"] if isinstance(obs, dict) else obs
-        assert np.array_equal(obs, p.mirror_frame(160, 120)[0])
-        assert np.array_equal(p.ref.render_top_view(), p.mirror_top_view(160, 120))
-        assert p.ref_visible() == p.mirror_visible(160, 120)
+    m = Mirror(level, False, obs_width=160, obs_height=120)
+    frames = load_frames(recorded, "views %s" % level)
+    assert frames
+    for f in replay(m, frames):
+        assert np.array_equal(frame_digest(m.mirror_frame(160, 120)[0]), f["digest"][0])
+        assert np.array_equal(frame_digest(m.mirror_top_view(160, 120)), f["digest"][1])
+        assert sum(1 << e for e in m.mirror_visible(160, 120)) == f["vis"]
 
 
-@needs_reference
-def test_reference_human_view_is_16_samples_and_equals_mirror(softgl_lib):
+def test_reference_human_view_is_16_samples_and_equals_mirror(softgl_lib, recorded):
     """render() with render_mode="rgb_array": the reference's vis_fb = FrameBuffer(window_width, window_height, 16)
     (miniworld.py:518); under the recording GL (GL_MAX_SAMPLES = 16) the frame it returns is a 16-sample frame and
     equals the mirror rendered with the D3D 16-sample pattern -- agent view and map view."""
-    from oracle.stream_check import Pair
     for view in ("agent", "top"):
-        p = Pair("MiniWorld-Hallway-v0", False, render_mode="rgb_array", window_width=160, window_height=120, view=view)
-        p.reset(5)
-        p.step(2)
-        got = p.ref.render()
-        fr = ref_stub.recorder.frames[-1]
-        assert fr.samples == 16 and got.shape == (120, 160, 3)
-        want = p.mirror_frame(160, 120, 16)[0] if view == "agent" else p.mirror_top_view(160, 120, 16)
-        assert np.array_equal(got, want)
+        assert recorded["human_%s_samples" % view] == 16
+        m = Mirror("MiniWorld-Hallway-v0", False, render_mode="rgb_array", window_width=160, window_height=120, view=view)
+        for f in replay(m, load_frames(recorded, "human %s" % view)):
+            want = m.mirror_frame(160, 120, 16)[0] if view == "agent" else m.mirror_top_view(160, 120, 16)
+            assert want.shape == (120, 160, 3)
+            assert np.array_equal(frame_digest(want), f["digest"][0]), view
 
 
-@needs_reference
-def test_reference_own_render_test_holds_on_the_recorded_stream():
+def test_reference_own_render_test_holds_on_the_recorded_stream(softgl_lib, recorded):
     """The one pixel-level statement the reference's test suite makes (tests/test_miniworld.py:17-38, Hallway,
     render_mode="rgb_array"): 0 < mean(obs) < 255, |mean(80x60 observation) - mean(800x600 human view)| < 5, and the
-    observation shapes -- evaluated on what the unmodified reference returns under the recording GL."""
-    env = ref_stub.make_reference_env("MiniWorld-Hallway-v0", record=True, render_mode="rgb_array")
-    for seed in (0, 1):
-        env.reset(seed=seed)
-        for _ in range(3):
-            obs, _, _, _, _ = env.step(0)
-        first_obs, _ = env.reset(seed=seed + 10)
-        first_render = env.render()
-        assert first_render.shape == (600, 800, 3) and ref_stub.recorder.frames[-1].samples == 16
+    observation shapes -- evaluated on what the unmodified reference returned under the recording GL, which the mirror
+    reproduces bit for bit."""
+    m = Mirror("MiniWorld-Hallway-v0", False, render_mode="rgb_array")
+    frames = load_frames(recorded, "render_test")
+    assert len(frames) == 2 and (recorded["render_test_samples"] == 16).all()
+    for f, second_shape in zip(replay(m, frames), recorded["render_test_second_obs_shape"]):
+        first_obs, first_render = m.mirror_frame()[0], m.mirror_frame(800, 600, 16)[0]
+        assert np.array_equal(frame_digest(first_obs), f["digest"][0])
+        assert np.array_equal(frame_digest(first_render), f["digest"][1])
+        assert first_render.shape == (600, 800, 3)
         m0, m1 = first_obs.mean(), first_render.mean()
         assert 0 < m0 < 255
         assert abs(m0 - m1) < 5, (m0, m1)
-        second_obs, _, _, _, _ = env.step(0)
-        assert first_obs.shape == env.observation_space.shape == second_obs.shape
+        space = tuple(recorded["render_test_observation_space_shape"])
+        assert first_obs.shape == space == m.mir.observation_space.shape == tuple(second_shape)
 
 
-@needs_reference
 def test_reference_light_is_directional():
     """(GLfloat * 4)(*self.light_pos + [1]) with an ndarray light_pos passes THREE values, each + 1, and leaves w = 0
-    (miniworld.py:1031, params.py:45-46): LIGHT0 is a directional light along light_pos + 1."""
-    env = ref_stub.make_reference_env("MiniWorld-OneRoom-v0", record=True)
-    env.reset(seed=3)
-    fr = ref_stub.recorder.frames[-1]
-    assert isinstance(env.light_pos, np.ndarray)
-    assert np.array_equal(fr.light["position"], np.array([1.0, 3.5, 1.0, 0.0], np.float32))
+    (miniworld.py:1031, params.py:45-46): LIGHT0 is a directional light along light_pos + 1.  The reference's recorded
+    glLightfv position after reset(seed=3) of OneRoom is what the pixel oracle passes for the mirror."""
+    want = np.load(os.path.join(GOLDEN, "mirror_frames.npz"))["light_position_oneroom_seed3"]
+    assert np.array_equal(want, np.array([1.0, 3.5, 1.0, 0.0], np.float32))
+    m = Mirror("MiniWorld-OneRoom-v0", False)
+    m.reset_mirror(3)
+    assert isinstance(m.mir.light_pos, np.ndarray)
+    assert softgl.light_position(m.mir) == list(want)
 
 
 @pytest.mark.parametrize("name", stream_cases())

@@ -1,5 +1,4 @@
-"""Host-side world generation (miniworld_b200.world / envs) against the reference:
-committed golden fixtures always, the live reference too where /root/reference exists."""
+"""Host-side world generation (miniworld_b200.world / envs) against the reference's, stored as golden fixtures."""
 import numpy as np
 import pytest
 
@@ -31,64 +30,40 @@ def test_reset_matches_reference_golden(name):
 
 
 def test_live_reference_world_generation():
-    from oracle import ref_stub
-    if not ref_stub.reference_available():
-        pytest.skip("/root/reference not present on this box")
-    for eid, kw in [("MiniWorld-FourRooms-v0", {}), ("MiniWorld-FourRooms-v0", {"domain_rand": True}),
-                    ("MiniWorld-PickupObjects-v0", {"domain_rand": True}), ("MiniWorld-Hallway-v0", {})]:
-        ref = ref_stub.make_reference_env(eid, **kw)
-        mine = LEVELS[eid](device=None, **kw)
-        for seed in (5, 6, 7):
-            ref.reset(seed=seed)
-            mine.reset(seed=seed)
-            for a, b in zip(ref.entities, mine.entities):
-                assert np.array_equal(np.asarray(a.pos, float), np.asarray(b.pos, float)) and a.dir == b.dir
-                assert a.radius == b.radius and type(a.radius) is type(b.radius)
-            assert np.array_equal(ref.wall_segs, mine.wall_segs)
-            for ra, rb in zip(ref.rooms, mine.rooms):
-                assert np.array_equal(ra.wall_verts, rb.wall_verts) and np.array_equal(ra.wall_texcs, rb.wall_texcs)
-                assert np.array_equal(ra.floor_texcs, rb.floor_texcs) and np.array_equal(ra.wall_norms, rb.wall_norms)
-            assert ref.np_random.random() == mine.np_random.random()
-
-
-def test_reference_level_file_runs_on_this_engine_api():
-    """Drop-in check: the reference's own envs/fourrooms.py source, imported against this
-    package's MiniWorldEnv / Box, generates the identical world."""
-    import importlib.util
+    """reset(seed) of the reference levels (tests/golden/worldgen_reference.npz, oracle/gen_mirror_golden.py) vs this
+    package: entity poses and radii (value and Python type), wall segments, room geometry and the next draw of
+    np_random."""
     import os
-    import sys
-    import types
-    path = "/root/reference/miniworld/envs/fourrooms.py"
-    if not os.path.exists(path):
-        pytest.skip("/root/reference not present on this box")
-    import miniworld_b200
-    from miniworld_b200 import _gym, entity, world
-    saved = {k: sys.modules.get(k) for k in ("miniworld", "miniworld.entity", "miniworld.miniworld", "gymnasium")}
-    if saved["miniworld"] is not None:
-        pytest.skip("the real `miniworld` package is imported in this process")
-    try:
-        pkg = types.ModuleType("miniworld")
-        sys.modules.update({"miniworld": pkg, "miniworld.entity": entity, "miniworld.miniworld": world})
-        if not _gym.HAVE_GYMNASIUM:
-            shim = types.ModuleType("gymnasium")
-            shim.spaces, shim.utils = _gym.spaces, _gym.utils
-            sys.modules["gymnasium"] = shim
-        spec = importlib.util.spec_from_file_location("ref_fourrooms", path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        theirs = mod.FourRooms(device=None)
-        ours = miniworld_b200.envs.FourRooms(device=None)
-        theirs.reset(seed=3)
-        ours.reset(seed=3)
-        assert np.array_equal(theirs.agent.pos, ours.agent.pos) and theirs.agent.dir == ours.agent.dir
-        assert np.array_equal(theirs.box.pos, ours.box.pos)
-        assert np.array_equal(theirs.wall_segs, ours.wall_segs)
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
+    from conftest import GOLDEN
+    from oracle.gen_mirror_golden import WORLDGEN_CASES, WORLDGEN_SEEDS
+    with np.load(os.path.join(GOLDEN, "worldgen_reference.npz")) as z:
+        ref = {k: z[k] for k in z.files}
+
+    def take(key, n):
+        """The next n rows of ref[key]."""
+        at = cursor.get(key, 0)
+        cursor[key] = at + n
+        return ref[key][at:at + n]
+
+    cursor, j, r = {}, 0, 0
+    for eid, kw in WORLDGEN_CASES:
+        mine = LEVELS[eid](device=None, **kw)
+        for seed in WORLDGEN_SEEDS:
+            mine.reset(seed=seed)
+            n = int(ref["n_ents"][j])
+            assert len(mine.entities) == n, (eid, kw, seed)
+            pos, dirs, radius, rtype = take("ent_pos", n), take("ent_dir", n), take("ent_radius", n), take("ent_radius_type", n)
+            for e, b in enumerate(mine.entities):
+                assert np.array_equal(pos[e], np.asarray(b.pos, float)) and dirs[e] == b.dir
+                assert radius[e] == b.radius and rtype[e] == type(b.radius).__name__
+            assert np.array_equal(take("wall_segs", int(ref["n_wall_segs"][j])), mine.wall_segs)
+            assert len(mine.rooms) == ref["n_rooms"][j]
+            for rb in mine.rooms:
+                for a, rows in zip(("wall_verts", "wall_texcs", "floor_texcs", "wall_norms"), ref["n_room_rows"][r]):
+                    assert np.array_equal(take(a, int(rows)), getattr(rb, a)), (eid, kw, seed, a)
+                r += 1
+            assert ref["next_random"][j] == mine.np_random.random()
+            j += 1
 
 
 @pytest.mark.parametrize("name", ["fourrooms", "hallway", "mazes3"])
