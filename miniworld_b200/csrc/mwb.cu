@@ -86,7 +86,6 @@ struct WorldUpload {   // AoS image of one env's dynamic state (host <-> device 
   mwb_rng_state rng;
 };
 
-#define MWB_MAX_D2H_CHUNKS 32
 #define MWB_DEFAULT_D2H_CHUNKS 16   // measured on B200 / PCIe 5: 4 -> 1.43 M, 8 -> 1.48 M, 16 -> 1.50 M env-steps/s end to end
 
 struct mwb_handle {
@@ -116,8 +115,6 @@ struct mwb_handle {
   bool have_params, have_protos, have_template;
   bool profiling;
   bool frames_copied;
-  int k2_variant;
-  int k2_flags;                   // MWB_K2_* measurement switches (env MWB_K2_FLAGS)
   int obs_peer_hint;              // mwb_set_obs_peer: 1 / 0 = the caller says where observations go, -1 = look it up
   const void* peer_checked;       // last observation pointer whose home device was looked up, and the answer
   bool peer_result;
@@ -128,8 +125,7 @@ struct mwb_handle {
   int k2_parts;                   // blocks per env frame (1 at 80x60, 4 at 160x120)
 #ifndef MWB_HOSTSIM
   cudaStream_t copy_stream;
-  cudaEvent_t chunk_done[MWB_MAX_D2H_CHUNKS], copies_done;
-  int d2h_chunks;                 // pieces a host-destination frame batch is rendered + copied in
+  cudaEvent_t chunk_done[MWB_DEFAULT_D2H_CHUNKS], copies_done;   // one per piece a host-destination frame batch is rendered + copied in
 #endif
 #ifndef MWB_HOSTSIM
   std::vector<cudaEvent_t> ev_k1, ev_k2;   // start/stop pairs
@@ -370,7 +366,6 @@ __global__ void seed_kernel(DevState S, const WorldUpload* u, int n) {
 #else
 // host simulator: sequential stand-in for mesh_setup_kernel + render_kernel built from the
 // same MWB_DEV functions
-static long long g_tile[6];   // half-tiles, bbox hits, after edge rejection, full covers, culled by an occluder, tiles with one
 struct VecTris {
   const TriRec* t;
   const TriRec& operator()(uint32_t slot) const { return t[slot]; }
@@ -429,50 +424,16 @@ static void hostsim_render_t(const DevState& S, const RenderAssets& A, const Vie
       tris.push_back(rec);
       pairable.push_back(0);
     }
-    const bool use_pairs = !getenv("MWB_HS_NOPAIRS");
-    // test-only experiment: visit triangles front to back (MWB_HS_SORT=1); slots keep draw order
+    // visit the triangles front to back by their nearest possible depth, as K2 does; slots keep draw order
     std::vector<int> order(tris.size());
-    for (size_t j = 0; j < tris.size(); ++j) order[j] = (int)j;
-    if (!getenv("MWB_HS_NOSORT")) {
-      std::vector<float> zmin(tris.size());
-      for (size_t j = 0; j < tris.size(); ++j) {
-        const TriRec& t = tris[j];
-        float x0 = (float)(t.bx & 0xFFFF), x1 = (float)((t.bx >> 16) + 1), y0 = (float)(t.by & 0xFFFF), y1 = (float)((t.by >> 16) + 1);
-        zmin[j] = t.Zc + fminf(t.Za * x0, t.Za * x1) + fminf(t.Zb * y0, t.Zb * y1);
-      }
-      std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return zmin[a] < zmin[b]; });
+    std::vector<float> zmin(tris.size());
+    for (size_t j = 0; j < tris.size(); ++j) {
+      const TriRec& t = tris[j];
+      float x0 = (float)(t.bx & 0xFFFF), x1 = (float)((t.bx >> 16) + 1), y0 = (float)(t.by & 0xFFFF), y1 = (float)((t.by >> 16) + 1);
+      zmin[j] = t.Zc + fminf(t.Za * x0, t.Za * x1) + fminf(t.Zb * y0, t.Zb * y1);
+      order[j] = (int)j;
     }
-    if (getenv("MWB_HS_TILESTATS")) {   // test-only: how the half-tile level tests of K2 would triage this frame
-      for (int ty0 = 0; ty0 < H; ty0 += 4)
-        for (int tx0 = 0; tx0 < W; tx0 += 8) {
-          g_tile[0]++;
-          float occl = 65535.0f;
-          std::vector<float> zn;
-          for (size_t j = 0; j < tris.size(); ++j) {
-            const TriRec& t = tris[j];
-            const int bx0 = t.bx & 0xFFFF, bx1 = t.bx >> 16, by0 = t.by & 0xFFFF, by1 = t.by >> 16;
-            if (!(bx0 <= tx0 + 7 && bx1 >= tx0 && by0 <= ty0 + 3 && by1 >= ty0)) continue;
-            g_tile[1]++;
-            const float fx0 = (float)tx0, fy0 = (float)ty0;
-            bool hit = true, covers = true;
-            for (int k = 0; k < 3; ++k) {
-              const float e = t.A[k] * fx0 + t.B[k] * fy0;
-              if (e + t.K[k] < 0.0f) hit = false;
-              covers = covers && e + t.C[k] - t.R[k] + 8.0f * fminf(t.A[k], 0.0f) + 4.0f * fminf(t.B[k], 0.0f) > 0.0f;
-            }
-            if (!hit) continue;
-            g_tile[2]++;
-            const float zb = t.Za * fx0 + t.Zb * fy0, zmin = zb + t.Kz;
-            const float zmax = zb + t.Zc + t.Zr + 8.0f * fmaxf(t.Za, 0.0f) + 4.0f * fmaxf(t.Zb, 0.0f);
-            const float chi = zmax * 65535.0f + 1.5f;
-            zn.push_back(zmin * 65535.0f - 1.0f);
-            if (covers) g_tile[3]++;
-            if (covers && zmin >= 0.0f && zmax <= 1.0f && chi < 65535.0f) occl = fminf(occl, chi);
-          }
-          if (occl < 65535.0f) g_tile[5]++;
-          for (size_t k = 0; k < zn.size(); ++k) if (zn[k] > occl) g_tile[4]++;
-        }
-    }
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return zmin[a] < zmin[b]; });
     VecTris fetch{tris.data()};
     for (int py = 0; py < H; ++py)
       for (int px = 0; px < W; ++px) {
@@ -482,7 +443,7 @@ static void hostsim_render_t(const DevState& S, const RenderAssets& A, const Vie
           const int j = order[jj];
           const TriRec& t = tris[j];
           if ((t.bx & 0xFFFF) > px || (t.bx >> 16) < px || (t.by & 0xFFFF) > py || (t.by >> 16) < py) continue;
-          const TriRec* partner = use_pairs && pairable[j] ? &tris[j ^ 1] : nullptr;
+          const TriRec* partner = pairable[j] ? &tris[j ^ 1] : nullptr;
           if (classify_pixel<MSAA>(load_class(&t), j, px, py, P, partner, (j & 1) ? 1 : 2) == 0) continue;
           if (P.mode == MWB_PX_LAZY) {     // materialise the lazily held triangle (both halves of a lazily held pair) first
             raster_pixel<MSAA>(load_hot(&tris[P.lazy_slot]), P.lazy_slot, px, py, P.keys, P.kmax);
@@ -564,7 +525,7 @@ static int k2_frame_stage_bytes(const mwb_handle* h) {
   if (h->k2_parts != 1 && (h->obs_format != MWB_OBS_HWC_U8 || (H & 3) != 0)) return 0;
   // Staging pays only when the stores leave the GPU (peer memory of rank 0: full 16-byte address-ordered stores
   // instead of 8-byte row segments, 52 % -> 89 % weak-scaling efficiency on 8 GPUs); for local HBM it costs 6 %.
-  if ((h->k2_flags & MWB_K2_NO_FRAME_STAGE) || !(h->obs_is_peer || (h->k2_flags & MWB_K2_FORCE_FRAME_STAGE))) return 0;
+  if (!h->obs_is_peer) return 0;
   // not at the price of a resident block: three blocks per SM (+ 1 KB each for the system) must still fit in 227 KB
   const size_t per_block = (size_t)k2_list_bytes(h) + bytes + (size_t)h->k2_static_smem + 1024;
   if (3 * per_block > 232448) return 0;
@@ -572,26 +533,25 @@ static int k2_frame_stage_bytes(const mwb_handle* h) {
 }
 static int k2_smem_bytes(const mwb_handle* h) { return k2_list_bytes(h) + k2_frame_stage_bytes(h); }
 
+// K2's instantiation for a sample count (1, 4, 8 or 16)
+static decltype(&render_kernel<8>) k2_kernel(int msaa) {
+  switch (msaa) {
+    case 1: return render_kernel<1>;
+    case 4: return render_kernel<4>;
+    case 16: return render_kernel<16>;
+    default: return render_kernel<8>;
+  }
+}
+
 // The opt-in for large dynamic shared memory is an attribute of the kernel FUNCTION (per device), not of a
 // handle: several handles with different triangle capacities share it, so it is only ever raised.
-static int g_k2_smem[16][3] = {};
+static int g_k2_smem[16] = {};
 static int ensure_k2_smem(mwb_handle* h, int smem) {
   const int dev = h->cfg.device & 15;
-  if (smem <= g_k2_smem[dev][h->k2_variant]) return 0;
-#define MWB_K2_ATTR(T, B, D)                                                                                               \
-  (cudaFuncSetAttribute(render_kernel<1, T, B, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess ||    \
-   cudaFuncSetAttribute(render_kernel<4, T, B, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess ||    \
-   cudaFuncSetAttribute(render_kernel<8, T, B, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess ||    \
-   cudaFuncSetAttribute(render_kernel<16, T, B, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess)
-  bool bad;
-  switch (h->k2_variant) {
-    case 0: bad = MWB_K2_ATTR(256, 3, true); break;
-    case 1: bad = MWB_K2_ATTR(320, 3, true); break;
-    default: bad = MWB_K2_ATTR(512, 2, true); break;
-  }
-#undef MWB_K2_ATTR
-  if (bad) return -1;
-  g_k2_smem[dev][h->k2_variant] = smem;
+  if (smem <= g_k2_smem[dev]) return 0;
+  for (int msaa : {1, 4, 8, 16})
+    if (cudaFuncSetAttribute(k2_kernel(msaa), cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return -1;
+  g_k2_smem[dev] = smem;
   return 0;
 }
 #endif
@@ -646,13 +606,7 @@ extern "C" int mwb_create(const mwb_config* cfg, mwb_handle** out) {
     delete h;
     return fail(MWB_ECUDA, "cudaStreamCreate failed");
   }
-  for (int c = 0; c < MWB_MAX_D2H_CHUNKS; ++c) cudaEventCreateWithFlags(&h->chunk_done[c], cudaEventDisableTiming);
-  {
-    const char* v = getenv("MWB_D2H_CHUNKS");   // tuning knob
-    h->d2h_chunks = v ? atoi(v) : MWB_DEFAULT_D2H_CHUNKS;
-    if (h->d2h_chunks < 1) h->d2h_chunks = 1;
-    if (h->d2h_chunks > MWB_MAX_D2H_CHUNKS) h->d2h_chunks = MWB_MAX_D2H_CHUNKS;
-  }
+  for (int c = 0; c < MWB_DEFAULT_D2H_CHUNKS; ++c) cudaEventCreateWithFlags(&h->chunk_done[c], cudaEventDisableTiming);
   cudaEventCreateWithFlags(&h->copies_done, cudaEventDisableTiming);
   cudaEventCreateWithFlags(&h->last_done, cudaEventDisableTiming);
   h->last_stream = h->stream;
@@ -745,36 +699,12 @@ extern "C" int mwb_create(const mwb_config* cfg, mwb_handle** out) {
   }
   // static quads are staged in shared memory (TMA bulk copy) when they fit in 16 KB; the
   // quad capacity is kept even so that every env's block starts 16-byte aligned
-  {
-    // tuning knob: 0 = 320 threads x 3 blocks/SM, warps stride over the half-tiles; 1 = same, warps claim
-    // half-tiles from a shared counter (default: -9 % kernel time on B200); 2 = 512 threads x 2 blocks/SM
-    const char* v = getenv("MWB_K2_VARIANT");
-    h->k2_variant = v ? atoi(v) : MWB_K2_DEFAULT_VARIANT;
-    if (h->k2_variant < 0 || h->k2_variant > 2) h->k2_variant = MWB_K2_DEFAULT_VARIANT;
-    const char* f = getenv("MWB_K2_FLAGS");
-    h->k2_flags = f ? atoi(f) : (MWB_K2_LISTS | MWB_K2_PAIRS);
-  }
   h->stage_bytes = (int)(((size_t)cfg->max_quads * sizeof(mwb_quad) + 15) & ~(size_t)15);
   if (h->stage_bytes > MWB_STAGE_QUAD_BYTES_HOST) h->stage_bytes = 0;
 #ifndef MWB_HOSTSIM
   {
     cudaFuncAttributes fa;
-    cudaError_t e;
-    switch (h->k2_variant) {
-      case 0: e = cfg->msaa_samples == 16 ? cudaFuncGetAttributes(&fa, render_kernel<16, 256, 3, true>)
-                : cfg->msaa_samples == 8 ? cudaFuncGetAttributes(&fa, render_kernel<8, 256, 3, true>)
-                : cfg->msaa_samples == 4 ? cudaFuncGetAttributes(&fa, render_kernel<4, 256, 3, true>)
-                                         : cudaFuncGetAttributes(&fa, render_kernel<1, 256, 3, true>); break;
-      case 1: e = cfg->msaa_samples == 16 ? cudaFuncGetAttributes(&fa, render_kernel<16, 320, 3, true>)
-                : cfg->msaa_samples == 8 ? cudaFuncGetAttributes(&fa, render_kernel<8, 320, 3, true>)
-                : cfg->msaa_samples == 4 ? cudaFuncGetAttributes(&fa, render_kernel<4, 320, 3, true>)
-                                         : cudaFuncGetAttributes(&fa, render_kernel<1, 320, 3, true>); break;
-      default: e = cfg->msaa_samples == 16 ? cudaFuncGetAttributes(&fa, render_kernel<16, 512, 2, true>)
-                : cfg->msaa_samples == 8 ? cudaFuncGetAttributes(&fa, render_kernel<8, 512, 2, true>)
-                 : cfg->msaa_samples == 4 ? cudaFuncGetAttributes(&fa, render_kernel<4, 512, 2, true>)
-                                          : cudaFuncGetAttributes(&fa, render_kernel<1, 512, 2, true>); break;
-    }
-    if (e == cudaSuccess) {
+    if (cudaFuncGetAttributes(&fa, k2_kernel(S.msaa)) == cudaSuccess) {
       h->k2_static_smem = (int)fa.sharedSizeBytes;
     } else {
       cudaGetLastError();
@@ -787,20 +717,11 @@ extern "C" int mwb_create(const mwb_config* cfg, mwb_handle** out) {
     return fail(MWB_ECUDA, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed");
   }
   if (getenv("MWB_DEBUG")) {
-    int nb = 0;
-    switch (h->k2_variant) {
-      case 0: cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, render_kernel<8, 256, 3, true>, 320, smem); break;
-      case 1: cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, render_kernel<8, 320, 3, true>, 320, smem); break;
-      default: cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, render_kernel<8, 512, 2, true>, 512, smem); break;
-    }
     const int launch_smem = k2_smem_bytes(h);
-    switch (h->k2_variant) {
-      case 0: cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, render_kernel<8, 256, 3, true>, 256, launch_smem); break;
-      case 1: cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, render_kernel<8, 320, 3, true>, 320, launch_smem); break;
-      default: cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, render_kernel<8, 512, 2, true>, 512, launch_smem); break;
-    }
-    fprintf(stderr, "[mwb] K2 variant %d: dynamic smem %d B (local destination), parts %d, resident blocks/SM (8x MSAA) %d\n",
-            h->k2_variant, launch_smem, h->k2_parts, nb);
+    int nb = 0;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k2_kernel(S.msaa), MWB_K2_THREADS, launch_smem);
+    fprintf(stderr, "[mwb] K2 %d threads, %dx MSAA: dynamic smem %d B (local destination), parts %d, resident blocks/SM %d\n",
+            MWB_K2_THREADS, S.msaa, launch_smem, h->k2_parts, nb);
   }
 #endif
   *out = h;
@@ -825,7 +746,7 @@ extern "C" int mwb_destroy(mwb_handle* h) {
   cudaStreamSynchronize(h->copy_stream);
   for (cudaEvent_t e : h->ev_k1) cudaEventDestroy(e);
   for (cudaEvent_t e : h->ev_k2) cudaEventDestroy(e);
-  for (int c = 0; c < MWB_MAX_D2H_CHUNKS; ++c) cudaEventDestroy(h->chunk_done[c]);
+  for (int c = 0; c < MWB_DEFAULT_D2H_CHUNKS; ++c) cudaEventDestroy(h->chunk_done[c]);
   cudaEventDestroy(h->copies_done);
   cudaEventDestroy(h->last_done);
   cudaStreamDestroy(h->copy_stream);
@@ -844,15 +765,6 @@ extern "C" int64_t mwb_overflow_count(mwb_handle* h) {
   if (d2h(&v, h->d_overflow, sizeof(int), h->stream) != 0 || sync_stream(h->stream) != 0) return -1;
   return v;
 }
-#ifdef MWB_HOSTSIM
-extern "C" void hs_counters(long long* out, int reset) {
-  for (int k = 0; k < 6; ++k) { out[k] = g_cnt[k]; if (reset) g_cnt[k] = 0; }
-}
-extern "C" void hs_tile_counters(long long* out, int reset) {
-  for (int k = 0; k < 6; ++k) { out[k] = g_tile[k]; if (reset) g_tile[k] = 0; }
-}
-#endif
-
 extern "C" int mwb_abi_sizes(int32_t* out, int cap) {
   const int32_t sz[] = {(int32_t)sizeof(mwb_config), (int32_t)sizeof(mwb_params), (int32_t)sizeof(mwb_tex_desc),
                         (int32_t)sizeof(mwb_mesh_desc), (int32_t)sizeof(mwb_room), (int32_t)sizeof(mwb_quad),
@@ -871,6 +783,92 @@ static int replace_buf(void** slot, const void* host, size_t bytes, stream_t s) 
   if (bytes && h2d(*slot, host, bytes, s) != 0) return fail(MWB_ECUDA, "upload failed");
   return sync_stream(s) == 0 ? 0 : fail(MWB_ECUDA, "sync failed");
 }
+
+#ifndef MWB_HOSTSIM
+// Atlas for K2's tld4 path: every mip level of every texture in ONE 2-D CUDA array (so that the texture handle is
+// the same for every lane whatever surface / LOD its pixel needs), each level framed by a one-texel wrapped border.
+// Shelf packing, tallest first; width 4096, height the next power of two.  Atlases are shared between the handles of
+// a process (keyed by device + a hash of the texel pool): building one costs ~0.1-0.5 s.  Returns null when the
+// atlas would be taller than 32768 rows or a CUDA call fails; K2 then reads the texel pool instead (the path the
+// host simulator always takes).
+static AtlasEntry* build_atlas(int device, const std::vector<TexDev>& td, const std::vector<uint32_t>& pool) {
+  const int n = (int)td.size();
+  uint64_t hash = 1469598103934665603ull;
+  auto mix = [&hash](uint64_t v) { hash = (hash ^ v) * 1099511628211ull; };
+  mix((uint64_t)n);
+  for (int t = 0; t < n; ++t) { mix((uint64_t)td[t].w << 32 | (uint32_t)td[t].h); mix((uint64_t)td[t].nlev); }
+  for (size_t k = 0; k + 1 < pool.size(); k += 2) mix((uint64_t)pool[k] << 32 | pool[k + 1]);
+  for (AtlasEntry* c : g_atlases)
+    if (c->device == device && c->hash == hash && c->texels == pool.size()) return c;
+  struct Item { int t, l, w, hgt; };
+  std::vector<Item> items;
+  for (int t = 0; t < n; ++t)
+    for (int l = 0; l < td[t].nlev; ++l) items.push_back({t, l, td[t].lw[l] + 2, td[t].lh[l] + 2});
+  std::stable_sort(items.begin(), items.end(), [](const Item& a, const Item& b) { return a.hgt > b.hgt; });
+  const int AW = 4096;
+  int cx = 0, cy = 0, shelf = 0;
+  std::vector<std::pair<int, int>> at(items.size());
+  for (size_t k = 0; k < items.size(); ++k) {
+    if (cx + items[k].w > AW) { cx = 0; cy += shelf; shelf = 0; }
+    at[k] = {cx, cy};
+    cx += items[k].w;
+    shelf = std::max(shelf, items[k].hgt);
+  }
+  int AH = 1;
+  while (AH < cy + shelf) AH <<= 1;
+  if (AH > 32768) return nullptr;
+  AtlasEntry* e = new AtlasEntry();
+  e->device = device;
+  e->hash = hash;
+  e->texels = pool.size();
+  e->refs = 0;
+  e->arr = nullptr;
+  e->obj = 0;
+  e->ax.assign((size_t)n * MWB_MAX_LEVELS, 0.0f);
+  e->ay.assign((size_t)n * MWB_MAX_LEVELS, 0.0f);
+  std::vector<uint32_t> atlas((size_t)AW * AH, 0u);
+  for (size_t k = 0; k < items.size(); ++k) {
+    const Item& it = items[k];
+    const int lw = it.w - 2, lh = it.hgt - 2;
+    const uint32_t* src = pool.data() + td[it.t].off[it.l];
+    for (int y = -1; y <= lh; ++y) {
+      uint32_t* dst = &atlas[(size_t)(at[k].second + 1 + y) * AW + at[k].first];
+      const uint32_t* row = src + (size_t)((y + lh) % lh) * lw;
+      dst[0] = row[lw - 1];
+      memcpy(dst + 1, row, (size_t)lw * 4);
+      dst[lw + 1] = row[0];
+    }
+    e->ax[(size_t)it.t * MWB_MAX_LEVELS + it.l] = (float)(at[k].first + 1);
+    e->ay[(size_t)it.t * MWB_MAX_LEVELS + it.l] = (float)(at[k].second + 1);
+  }
+  const cudaChannelFormatDesc fmt = cudaCreateChannelDesc<uchar4>();
+  bool ok = cudaMallocArray(&e->arr, &fmt, AW, AH, cudaArrayTextureGather) == cudaSuccess;
+  if (ok) ok = cudaMemcpy2DToArray(e->arr, 0, 0, atlas.data(), (size_t)AW * 4, (size_t)AW * 4, AH, cudaMemcpyHostToDevice) == cudaSuccess;
+  if (ok) {
+    cudaResourceDesc rd;
+    memset(&rd, 0, sizeof(rd));
+    rd.resType = cudaResourceTypeArray;
+    rd.res.array.array = e->arr;
+    cudaTextureDesc tdesc;
+    memset(&tdesc, 0, sizeof(tdesc));
+    tdesc.addressMode[0] = tdesc.addressMode[1] = cudaAddressModeClamp;
+    tdesc.filterMode = cudaFilterModePoint;
+    tdesc.readMode = cudaReadModeNormalizedFloat;
+    tdesc.normalizedCoords = 1;
+    ok = cudaCreateTextureObject(&e->obj, &rd, &tdesc, nullptr) == cudaSuccess;
+  }
+  if (!ok) {
+    cudaGetLastError();
+    if (e->arr) cudaFreeArray(e->arr);
+    delete e;
+    return nullptr;
+  }
+  e->iw = 1.0f / (float)AW;
+  e->ih = 1.0f / (float)AH;
+  g_atlases.push_back(e);
+  return e;
+}
+#endif
 
 // ------------------------------------------------------------------ ABI: assets
 extern "C" int mwb_upload_textures(mwb_handle* h, const mwb_tex_desc* descs, int n, const uint8_t* rgb) {
@@ -924,106 +922,19 @@ extern "C" int mwb_upload_textures(mwb_handle* h, const mwb_tex_desc* descs, int
     T.nlev = lev;
   }
 #ifndef MWB_HOSTSIM
-  // ---- atlas for K2's tld4 path: every mip level of every texture in ONE 2-D CUDA array (so that the texture
-  // handle is the same for every lane whatever surface / LOD its pixel needs), each level framed by a one-texel
-  // wrapped border.  Shelf packing, tallest first; width 4096, height the next power of two.  Atlases are shared
-  // between the handles of a process (keyed by device + a hash of the texel pool): building one costs ~0.1-0.5 s.
   release_texture_objects(h);
   h->A.atlas = 0ull;
-  {
-    const char* tm = getenv("MWB_K2_TMU");
-    if (!tm || atoi(tm) != 0) {
-      uint64_t hash = 1469598103934665603ull;
-      auto mix = [&hash](uint64_t v) { hash = (hash ^ v) * 1099511628211ull; };
-      mix((uint64_t)n);
-      for (int t = 0; t < n; ++t) { mix((uint64_t)td[t].w << 32 | (uint32_t)td[t].h); mix((uint64_t)td[t].nlev); }
-      for (size_t k = 0; k + 1 < pool.size(); k += 2) mix((uint64_t)pool[k] << 32 | pool[k + 1]);
-      AtlasEntry* e = nullptr;
-      for (AtlasEntry* c : g_atlases)
-        if (c->device == h->cfg.device && c->hash == hash && c->texels == pool.size()) e = c;
-      if (!e) {
-        struct Item { int t, l, w, hgt; };
-        std::vector<Item> items;
-        for (int t = 0; t < n; ++t)
-          for (int l = 0; l < td[t].nlev; ++l) items.push_back({t, l, td[t].lw[l] + 2, td[t].lh[l] + 2});
-        std::stable_sort(items.begin(), items.end(), [](const Item& a, const Item& b) { return a.hgt > b.hgt; });
-        const int AW = 4096;
-        int cx = 0, cy = 0, shelf = 0;
-        std::vector<std::pair<int, int>> at(items.size());
-        for (size_t k = 0; k < items.size(); ++k) {
-          if (cx + items[k].w > AW) { cx = 0; cy += shelf; shelf = 0; }
-          at[k] = {cx, cy};
-          cx += items[k].w;
-          shelf = std::max(shelf, items[k].hgt);
-        }
-        int AH = 1;
-        while (AH < cy + shelf) AH <<= 1;
-        if (AH <= 32768) {
-          e = new AtlasEntry();
-          e->device = h->cfg.device;
-          e->hash = hash;
-          e->texels = pool.size();
-          e->refs = 0;
-          e->arr = nullptr;
-          e->obj = 0;
-          e->ax.assign((size_t)n * MWB_MAX_LEVELS, 0.0f);
-          e->ay.assign((size_t)n * MWB_MAX_LEVELS, 0.0f);
-          std::vector<uint32_t> atlas((size_t)AW * AH, 0u);
-          for (size_t k = 0; k < items.size(); ++k) {
-            const Item& it = items[k];
-            const int lw = it.w - 2, lh = it.hgt - 2;
-            const uint32_t* src = pool.data() + td[it.t].off[it.l];
-            for (int y = -1; y <= lh; ++y) {
-              uint32_t* dst = &atlas[(size_t)(at[k].second + 1 + y) * AW + at[k].first];
-              const uint32_t* row = src + (size_t)((y + lh) % lh) * lw;
-              dst[0] = row[lw - 1];
-              memcpy(dst + 1, row, (size_t)lw * 4);
-              dst[lw + 1] = row[0];
-            }
-            e->ax[(size_t)it.t * MWB_MAX_LEVELS + it.l] = (float)(at[k].first + 1);
-            e->ay[(size_t)it.t * MWB_MAX_LEVELS + it.l] = (float)(at[k].second + 1);
-          }
-          const cudaChannelFormatDesc fmt = cudaCreateChannelDesc<uchar4>();
-          bool ok = cudaMallocArray(&e->arr, &fmt, AW, AH, cudaArrayTextureGather) == cudaSuccess;
-          if (ok) ok = cudaMemcpy2DToArray(e->arr, 0, 0, atlas.data(), (size_t)AW * 4, (size_t)AW * 4, AH, cudaMemcpyHostToDevice) == cudaSuccess;
-          if (ok) {
-            cudaResourceDesc rd;
-            memset(&rd, 0, sizeof(rd));
-            rd.resType = cudaResourceTypeArray;
-            rd.res.array.array = e->arr;
-            cudaTextureDesc tdesc;
-            memset(&tdesc, 0, sizeof(tdesc));
-            tdesc.addressMode[0] = tdesc.addressMode[1] = cudaAddressModeClamp;
-            tdesc.filterMode = cudaFilterModePoint;
-            tdesc.readMode = cudaReadModeNormalizedFloat;
-            tdesc.normalizedCoords = 1;
-            ok = cudaCreateTextureObject(&e->obj, &rd, &tdesc, nullptr) == cudaSuccess;
-          }
-          if (ok) {
-            e->iw = 1.0f / (float)AW;
-            e->ih = 1.0f / (float)AH;
-            g_atlases.push_back(e);
-          } else {
-            cudaGetLastError();
-            if (e->arr) cudaFreeArray(e->arr);
-            delete e;
-            e = nullptr;                     // the pool path stays in use
-          }
-        }
+  if (AtlasEntry* e = build_atlas(h->cfg.device, td, pool)) {
+    e->refs++;
+    h->atlas = e;
+    for (int t = 0; t < n; ++t)
+      for (int l = 0; l < td[t].nlev; ++l) {
+        td[t].ax[l] = e->ax[(size_t)t * MWB_MAX_LEVELS + l];
+        td[t].ay[l] = e->ay[(size_t)t * MWB_MAX_LEVELS + l];
       }
-      if (e) {
-        e->refs++;
-        h->atlas = e;
-        for (int t = 0; t < n; ++t)
-          for (int l = 0; l < td[t].nlev; ++l) {
-            td[t].ax[l] = e->ax[(size_t)t * MWB_MAX_LEVELS + l];
-            td[t].ay[l] = e->ay[(size_t)t * MWB_MAX_LEVELS + l];
-          }
-        h->A.atlas = (unsigned long long)e->obj;
-        h->A.atlas_iw = e->iw;
-        h->A.atlas_ih = e->ih;
-      }
-    }
+    h->A.atlas = (unsigned long long)e->obj;
+    h->A.atlas_iw = e->iw;
+    h->A.atlas_ih = e->ih;
   }
 #endif
   int rc = replace_buf(&h->tex_desc, td.data(), td.size() * sizeof(TexDev), h->stream);
@@ -1492,19 +1403,9 @@ static int launch_k2(mwb_handle* h, uint8_t* obs, float* depth, int env0, int co
   const K2Layout lay = k2_layout(h->smem_tris, h->tri_cap, h->stage_bytes, k2_halves_per_part(h->S.obs_w, h->S.obs_h, h->k2_parts), fstage);
   if (ensure_k2_smem(h, smem)) return fail(MWB_ECUDA, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed");
   prof_mark(h, h->ev_k2, s);
-#define MWB_LAUNCH_K2(M, T, B, D) render_kernel<M, T, B, D><<<count * h->k2_parts, T, smem, s>>>(h->S, h->A, h->view, h->obs_format, obs, depth, env0, h->k2_parts, h->tri_cap, h->stage_bytes, fstage, h->k2_flags, lay, h->d_overflow)
-#define MWB_LAUNCH_K2_MSAA(T, B, D)                 \
-  switch (h->S.msaa) {                              \
-    case 1: MWB_LAUNCH_K2(1, T, B, D); break;       \
-    case 4: MWB_LAUNCH_K2(4, T, B, D); break;       \
-    case 16: MWB_LAUNCH_K2(16, T, B, D); break;     \
-    default: MWB_LAUNCH_K2(8, T, B, D); break;      \
-  }
-  switch (h->k2_variant) {
-    case 0: MWB_LAUNCH_K2_MSAA(256, 3, true); break;
-    case 1: MWB_LAUNCH_K2_MSAA(320, 3, true); break;
-    default: MWB_LAUNCH_K2_MSAA(512, 2, true); break;
-  }
+  k2_kernel(h->S.msaa)<<<count * h->k2_parts, MWB_K2_THREADS, smem, s>>>(h->S, h->A, h->view, h->obs_format, obs, depth, env0,
+                                                                          h->k2_parts, h->tri_cap, h->stage_bytes, fstage, lay,
+                                                                          h->d_overflow);
   prof_mark(h, h->ev_k2, s);
   h->launches++;
   CK(cudaGetLastError());
@@ -1533,7 +1434,7 @@ static int launch_render(mwb_handle* h, uint8_t* obs, float* depth, stream_t s, 
   const int N = h->S.N;
   const size_t px = (size_t)h->S.obs_w * h->S.obs_h;
   const bool pipelined = (host_obs || host_depth) && N >= 256;
-  int chunks = pipelined ? h->d2h_chunks : 1;
+  int chunks = pipelined ? MWB_DEFAULT_D2H_CHUNKS : 1;
   while (chunks > 1 && N / chunks < 256) --chunks;   // keep every launch a few hundred blocks wide
   for (int c = 0; c < chunks; ++c) {
     const int e0 = (int)((long long)N * c / chunks), e1 = (int)((long long)N * (c + 1) / chunks);
@@ -1636,7 +1537,7 @@ extern "C" int mwb_render_obs(mwb_handle* h, uint8_t* obs, float* depth, void* s
 
 extern "C" int mwb_set_obs_peer(mwb_handle* h, int peer) {
   if (!h) return fail(MWB_EINVAL, "null handle");
-  h->obs_peer_hint = peer ? 1 : 0;
+  h->obs_peer_hint = peer < 0 ? -1 : (peer ? 1 : 0);
   return MWB_OK;
 }
 

@@ -5,18 +5,20 @@
 // OpenGL draw + MSAA resolve + glReadPixels round trip, for N environments per launch.
 //
 // Structure of one block (env i, 10 warps; big frames are cut into several blocks per env):
-//   A. a TMA bulk copy stages the env's static quads in shared memory while six threads evaluate the
-//      camera's glibc-exact sin / cos and another lays out the frame's draw list.
+//   A. a TMA bulk copy stages the env's static quads in shared memory while one thread builds the camera
+//      from the glibc-exact cos / sin frame_trig_kernel evaluated and another lays out the frame's draw list.
 //   B. geometry: one thread per triangle task (half of a static room quad or of a box face)
 //      transforms, lights and sets up its triangle; survivors of frustum / back-face culling
 //      are compacted IN DRAW ORDER into shared memory (shuffle prefix scan) -- the set-up
-//      triangles of rooms and boxes never touch HBM.  Mesh entities (thousands of triangles)
-//      arrive as per-entity lists prepared AND binned by half-tile by mesh_setup_kernel.
-//   C. raster: warps claim 8x4 half-tiles from a shared counter (lane = pixel).  Per chunk of 32
-//      triangles every lane tests one triangle's bbox / edge functions / nearest depth against the
-//      half-tile and a warp ballot yields its coverage list; each listed triangle is classified per
-//      pixel (lazy single-surface pixels), undecided (pixel, triangle) pairs go through an exact
-//      sample-parallel phase on (depth16, slot) keys in shared memory.
+//      triangles of rooms and boxes never touch HBM.  They are ranked front to back and filed into
+//      per-half-tile candidate lists.  Mesh entities (thousands of triangles) arrive as per-entity
+//      lists prepared AND binned by half-tile by mesh_setup_kernel.
+//   C. raster: warps claim 8x4 half-tiles from a shared counter (lane = pixel).  The hot path walks the
+//      half-tile's candidate list; mesh lists and half-tiles whose list overflowed fall back to a scan in
+//      chunks of 32 triangles, where every lane tests one triangle's bbox / edge functions / nearest depth
+//      against the half-tile and a warp ballot yields the survivors.  Each triangle is classified per
+//      pixel (lazy single-surface pixels, quad pairs), undecided (pixel, triangle) pairs go through an
+//      exact sample-parallel phase on (depth16, slot) keys in shared memory.
 //   D. resolve: each pixel shades the distinct triangles its samples see (perspective-
 //      correct Gouraud x trilinear texture), box-filters, converts to unorm8; the half-tile is
 //      transposed through shared memory and written as 8-byte row segments (or channel-first /
@@ -26,13 +28,7 @@
 #pragma once
 #include "raster_core.cuh"
 
-#define MWB_K2_DEFAULT_VARIANT 1
-
 #define MWB_TILE_CAP 16              // candidate triangles listed per half-tile; fuller half-tiles scan the lists
-#define MWB_K2_LISTS 1               // kernel flags (env MWB_K2_FLAGS, default all on): per-half-tile candidate lists,
-#define MWB_K2_PAIRS 2               // quad-pair lazy pixels
-#define MWB_K2_NO_FRAME_STAGE 4      // host side: never stage the whole frame in shared memory
-#define MWB_K2_FORCE_FRAME_STAGE 8   // host side: stage it even when the destination is local memory
 
 // K2's dynamic shared memory, in this order (host and kernel share the arithmetic):
 //   [triangle records (small levels)]
@@ -286,13 +282,14 @@ __global__ void depth_lut_kernel(float* __restrict__ lut) {
 }
 
 // ---- K2 --------------------------------------------------------------------------------
-// THREADS x MINB: block size and resident blocks per SM the kernel is compiled for (64 registers per thread);
-// DYN: warps claim half-tiles from a shared counter instead of striding, which evens out the per-warp work.
-template <int MSAA, int THREADS, int MINB, bool DYN>
-__global__ void __launch_bounds__(THREADS, MINB)
+// Block size and resident blocks per SM K2 is compiled for (64 registers per thread): the measured default.
+// 256 x 3 was slower; 512 x 2 was equal on config 3 and 6 % slower on config 4.
+constexpr int MWB_K2_THREADS = 320, MWB_K2_MIN_BLOCKS = 3;
+template <int MSAA>
+__global__ void __launch_bounds__(MWB_K2_THREADS, MWB_K2_MIN_BLOCKS)
 render_kernel(DevState S, RenderAssets A, ViewSpec view, int fmt, uint8_t* __restrict__ obs, float* __restrict__ depth, int env0,
-              int parts, int tri_cap, int stage_bytes, int frame_stage_bytes, int flags, K2Layout lay, int* __restrict__ overflow) {
-  constexpr int WARPS = THREADS / 32;
+              int parts, int tri_cap, int stage_bytes, int frame_stage_bytes, K2Layout lay, int* __restrict__ overflow) {
+  constexpr int THREADS = MWB_K2_THREADS, WARPS = THREADS / 32;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   // large frames are cut into `parts` blocks per env (each redoes the cheap geometry phase and
   // rasterises its share of the half-tiles), which evens out the load when few envs are resident
@@ -318,7 +315,6 @@ render_kernel(DevState S, RenderAssets A, ViewSpec view, int fmt, uint8_t* __res
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int W = S.obs_w, H = S.obs_h;
-  const bool use_lists = (flags & MWB_K2_LISTS) != 0, pairs = (flags & MWB_K2_PAIRS) != 0;   // measurement switches
 
   // static room quads of this env: staged into shared memory by one TMA bulk copy that overlaps
   // the camera set-up (fixed-layout levels: 56 quads = 7.6 KB); larger templates are read from L2
@@ -420,7 +416,7 @@ render_kernel(DevState S, RenderAssets A, ViewSpec view, int fmt, uint8_t* __res
     zkey[t] = T.Zc + fminf(T.Za * x0, T.Za * x1) + fminf(T.Zb * y0, T.Zb * y1);
   }
   if (tid == 0) {
-    if (DYN) next_half = h_begin + WARPS;
+    next_half = h_begin + WARPS;
     if (ntris > tri_cap) atomicAdd(overflow, 1);
     // segment table: smem-resident lists are contiguous in draw order; mesh lists live in HBM
     int smem_pos = 0, slot = 0;
@@ -544,19 +540,17 @@ render_kernel(DevState S, RenderAssets A, ViewSpec view, int fmt, uint8_t* __res
   uint32_t(*skeys)[32] = ws.keys;
   uint32_t* equeue = ws.items;
   // half-tiles in row-major order of 8x4 blocks: index h -> column h % tiles_x, row h / tiles_x
-  int half = h_begin + warp;            // (DYN: next_half was set with the segment table, several barriers ago)
+  // the first WARPS half-tiles go one to each warp; after that warps claim half-tiles from next_half (set with the
+  // segment table, several barriers ago), which evens out the per-warp work
+  int half = h_begin + warp;
 #pragma unroll 1
   while (half < h_end) {
     const int hrow = (int)(((float)half + 0.5f) * inv_tiles_x), hcol = half - hrow * tiles_x;   // exact: half < 2^20
     const int tx0 = hcol << 3, ty0 = hrow << 2;
     const int hl = half - h_begin;
-    if (DYN) {                 // claim the next half-tile now; the atomic's latency hides behind this one
-      int nxt = 0;
-      if (lane == 0) nxt = atomicAdd(&next_half, 1);
-      half = __shfl_sync(0xffffffffu, nxt, 0);
-    } else {
-      half += WARPS;
-    }
+    int nxt = 0;               // claim the next half-tile now; the atomic's latency hides behind this one
+    if (lane == 0) nxt = atomicAdd(&next_half, 1);
+    half = __shfl_sync(0xffffffffu, nxt, 0);
     const int px = tx0 + lx, py = ty0 + ly;
     PixelState<MSAA> P;
     pixel_init(P);
@@ -630,7 +624,7 @@ render_kernel(DevState S, RenderAssets A, ViewSpec view, int fmt, uint8_t* __res
     // ---- hot path: this half-tile's list of block-resident triangles (already tested against the half-tile, in
     // front-to-back order); every listed triangle is triaged at each lane's pixel (warp-uniform loop)
     const int n_cand = tile_cnt[hl];
-    const bool listed = use_lists && n_cand <= MWB_TILE_CAP;
+    const bool listed = n_cand <= MWB_TILE_CAP;
     if (listed) {
       const uint16_t* list = tile_list + hl * MWB_TILE_CAP;
       uint32_t mine = 0, mine_full = 0;
@@ -638,7 +632,7 @@ render_kernel(DevState S, RenderAssets A, ViewSpec view, int fmt, uint8_t* __res
       for (int q = 0; q < n_cand; ++q) {
         const int p = list[q];
         const ClassTri ct = load_class(tris + p);
-        const int cls = classify_pixel<MSAA>(ct, (int)tri_slot[p], px, py, P, pairs ? tris + (p ^ 1) : nullptr, (p & 1) ? 1 : 2);
+        const int cls = classify_pixel<MSAA>(ct, (int)tri_slot[p], px, py, P, tris + (p ^ 1), (p & 1) ? 1 : 2);
         if (cls) mine |= 1u << q;
         if (cls == 2) mine_full |= 1u << q;
       }
@@ -651,7 +645,7 @@ render_kernel(DevState S, RenderAssets A, ViewSpec view, int fmt, uint8_t* __res
       const Segment sg = segs[sgi];
       if (sg.count == 0 || (listed && sg.bbox == nullptr)) continue;
       if ((sg.bx & 0xFFFF) > tx0 + 7 || (sg.bx >> 16) < tx0 || (sg.by & 0xFFFF) > ty0 + 3 || (sg.by >> 16) < ty0) continue;
-      const bool pairable = pairs && sg.bbox == nullptr;   // resident lists hold quad pairs in adjacent records
+      const bool pairable = sg.bbox == nullptr;   // resident lists hold quad pairs in adjacent records
       // which triangles to visit: a binned mesh list only the triangles filed under this half-tile; else the whole list
       const uint16_t* ord = nullptr;
       int lo = 0, hi = sg.count;

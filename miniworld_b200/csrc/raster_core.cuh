@@ -393,27 +393,18 @@ MWB_DEV uint32_t max_key(const uint32_t (&keys)[MSAA]) {
 // slots ascend in draw order, so on equal codes the earlier draw keeps the sample).
 // `kmax` caches max(keys): a triangle whose nearest possible depth code over the pixel is
 // already behind every stored sample cannot win any GL_LESS test and is skipped.
-#ifdef MWB_HOSTSIM
-static long long g_cnt[6];   // test-only statistics: pairs, outside, zclip, occluded, sampled, changed
-#define MWB_COUNT(k) (++g_cnt[k])
-#else
-#define MWB_COUNT(k)
-#endif
-
 template <int MSAA>
 MWB_DEV void raster_pixel(const HotTri& t, int slot, int px, int py, uint32_t (&keys)[MSAA], uint32_t& kmax) {
-  MWB_COUNT(0);
   const float cx = (float)px + 0.5f, cy = (float)py + 0.5f;
   const float e0 = t.A[0] * cx + t.B[0] * cy + t.C[0];
   const float e1 = t.A[1] * cx + t.B[1] * cy + t.C[1];
   const float e2 = t.A[2] * cx + t.B[2] * cy + t.C[2];
-  if (e0 + t.R[0] < 0.0f || e1 + t.R[1] < 0.0f || e2 + t.R[2] < 0.0f) { MWB_COUNT(1); return; }   // certainly outside
+  if (e0 + t.R[0] < 0.0f || e1 + t.R[1] < 0.0f || e2 + t.R[2] < 0.0f) return;  // certainly outside
   const float zc = t.Za * cx + t.Zb * cy + t.Zc;
   const float zlo = zc - t.Zr;
-  if (zlo > 1.0f || zc + t.Zr < 0.0f) { MWB_COUNT(2); return; }                  // beyond far / before near
+  if (zlo > 1.0f || zc + t.Zr < 0.0f) return;                                 // beyond far / before near
   // smallest code any sample of this pixel can get (one code of slack for the rounding of z * 65535)
-  if (zlo * 65535.0f - 1.0f > (float)(kmax >> 16)) { MWB_COUNT(3); return; }    // certainly occluded
-  MWB_COUNT(4);
+  if (zlo * 65535.0f - 1.0f > (float)(kmax >> 16)) return;                    // certainly occluded
   const bool full = e0 - t.R[0] > 0.0f && e1 - t.R[1] > 0.0f && e2 - t.R[2] > 0.0f;   // certainly inside
   const float fx = (float)px, fy = (float)py;
   bool changed = false;
@@ -433,7 +424,7 @@ MWB_DEV void raster_pixel(const HotTri& t, int slot, int px, int py, uint32_t (&
       changed = true;
     }
   }
-  if (changed) { MWB_COUNT(5); kmax = max_key<MSAA>(keys); }
+  if (changed) kmax = max_key<MSAA>(keys);
 }
 
 // ---------------------------------------------------------------------------- shading
@@ -522,19 +513,18 @@ MWB_DEV ClassTri load_class(const TriRec* t) {
 template <int MSAA>
 MWB_DEV int classify_pixel(const ClassTri& t, int slot, int px, int py, PixelState<MSAA>& p, const TriRec* partner = nullptr,
                            int diag = 0) {
-  MWB_COUNT(0);
   if (slot == p.pair_skip) return 0;                      // already covered through its partner at this pixel
   const float cx = (float)px + 0.5f, cy = (float)py + 0.5f;
   const float e0 = t.A[0] * cx + t.B[0] * cy + t.C[0];
   const float e1 = t.A[1] * cx + t.B[1] * cy + t.C[1];
   const float e2 = t.A[2] * cx + t.B[2] * cy + t.C[2];
-  if (e0 + t.R[0] < 0.0f || e1 + t.R[1] < 0.0f || e2 + t.R[2] < 0.0f) { MWB_COUNT(1); return 0; }   // certainly outside
+  if (e0 + t.R[0] < 0.0f || e1 + t.R[1] < 0.0f || e2 + t.R[2] < 0.0f) return 0;      // certainly outside
   const float zc = t.Za * cx + t.Zb * cy + t.Zc;
   const float zlo = zc - t.Zr, zhi = zc + t.Zr;
-  if (zlo > 1.0f || zhi < 0.0f) { MWB_COUNT(2); return 0; }                           // certainly clipped away
+  if (zlo > 1.0f || zhi < 0.0f) return 0;                                             // certainly clipped away
   // depth codes any sample of this pixel can get lie in [clo, chi] (one code of slack each way)
   float clo = zlo * 65535.0f - 1.0f, chi = zhi * 65535.0f + 1.5f;
-  if (clo > pixel_bound(p)) { MWB_COUNT(3); return 0; }                               // certainly occluded
+  if (clo > pixel_bound(p)) return 0;                                                 // certainly occluded
   const bool in0 = e0 - t.R[0] > 0.0f, in1 = e1 - t.R[1] > 0.0f, in2 = e2 - t.R[2] > 0.0f;
   const bool full = in0 && in1 && in2;                                                // covers every sample
   bool pair = false;
@@ -556,7 +546,6 @@ MWB_DEV int classify_pixel(const ClassTri& t, int slot, int px, int py, PixelSta
       p.lazy_clo = clo;
       p.lazy_chi = chi;
       if (pair) p.pair_skip = slot ^ 1;
-      MWB_COUNT(5);
       return 0;
     }
   }

@@ -79,8 +79,6 @@ def _worker_one_gpu(rank, world, port, total, steps, q, flag_mode, level="MiniWo
     """Two processes on cuda:0: the peer buffer crosses a process boundary (CUDA IPC), not a GPU boundary."""
     sys.path.insert(0, ROOT)
     os.environ["MWB_FLAG_MODE"] = flag_mode
-    if staged:
-        os.environ["MWB_K2_FLAGS"] = "11"       # lists | pairs | force the frame stage although the destination is local
     import torch
     import torch.distributed as dist
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
@@ -94,6 +92,8 @@ def _worker_one_gpu(rank, world, port, total, steps, q, flag_mode, level="MiniWo
     ok = env.enable_peer_obs()
     frames = []
     if ok:
+        if staged:
+            env.local.engine.set_obs_peer(True)   # stage frames as for another GPU although the destination is local
         for t in range(steps):              # no synchronisation between the ranks inside the loop: the flags order it
             obs = env.step_peer(torch.as_tensor(acts_all[t, env.start:env.start + env.count], device="cuda"))
             if rank == 0:
